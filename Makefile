@@ -18,10 +18,10 @@ bench: build      ## BASELINE.json metric, one JSON line
 bench-reference:  ## the reference's algorithm on the host cores, same metric
 	$(PY) bench.py --impl reference
 
-reference:        ## install the unmodified reference into baseline/_ref (the --impl reference arm, the drop-in GPU test)
-	bash baseline/install_reference.sh
+reference:        ## install the unmodified reference into oracle/_ref (the --impl reference arm, the drop-in tests)
+	bash oracle/install_reference.sh $(PRYSM_REFERENCE)
 
-parity:           ## full-array parity report of C2..C5 against the reference's fp64 run (needs a B200 and baseline/_ref)
+parity:           ## full-array parity report of C2..C5 against the reference's fp64 run (needs a B200 and oracle/_ref)
 	$(PY) tools/parity_report.py
 
 sanitizer:        ## compute-sanitizer memcheck + racecheck over the small-size parity tests (needs a B200)

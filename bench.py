@@ -2,6 +2,7 @@
 """bench.py -- BASELINE.json metric: 2048x2048 pupil -> PSF propagations/sec.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--calls-per-step C] [--no-extras]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE configs[1], SURVEY.md 8d "C2"): one unit = `focus(pupil, Q=2)` of a 2048^2 complex64
@@ -12,8 +13,8 @@ SURVEY.md 8e).
 
 The JSON line carries: value (device-resident throughput, CUDA events, max over ranks), e2e (the same metric through
 `Wavefront(...).focus()` with pinned HOST buffers, H2D + D2H inside the timed region), roofline (algorithmic bytes /
-measured duration against the measured HBM peak), cpu_baseline (the unmodified reference from baseline/_ref on this
-box's host cores), clocks, and -- at every N -- the other BASELINE configs as extras:
+measured duration against the measured HBM peak), cpu_baseline (the unmodified reference from oracle/_ref on the
+host cores), clocks, and -- at every N -- the other BASELINE configs as extras:
   mdft_c3 (N = 1), c4_polychromatic (64 wavelengths sharded over the ranks, ONE NCCL reduce inside the timed region),
   c5_free_space (32-plane screened angular-spectrum chain + CZT final focus, one chain per rank).
 """
@@ -162,10 +163,10 @@ def bind_to_gpu_numa_node(local):
 # ---------------------------------------------------------------------------------------------------------------
 def reference_focus():
     """(callable pupil -> 4096^2 complex64 field, kind).  kind = "reference": the UNMODIFIED prysm installed in
-    baseline/_ref by baseline/install_reference.sh, driven through its own public API
+    oracle/_ref by oracle/install_reference.sh, driven through its own public API
     (Wavefront(...).focus(efl, Q=2), prysm/propagation/wavefront.py:478-504) at config.precision = 32.
     Fallback when that directory is missing: the oracle port of the same call ("port")."""
-    ref_dir = os.path.join(ROOT, 'baseline', '_ref')
+    ref_dir = os.path.join(ROOT, 'oracle', '_ref')
     if os.path.isdir(os.path.join(ref_dir, 'prysm')):
         sys.path.insert(0, ref_dir)
         from prysm.conf import config as pconfig
@@ -200,7 +201,7 @@ def cpu_focus_rate(run, seconds_budget, workers, pupils, min_reps=3):
 
 
 def run_reference(args):
-    """--impl reference: the reference's own CPU implementation of the path (unmodified prysm from baseline/_ref,
+    """--impl reference: the reference's own CPU implementation of the path (unmodified prysm from oracle/_ref,
     numpy + scipy.fft pocketfft), all host threads, same config / metric.  Rank 0 only."""
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
@@ -411,6 +412,24 @@ def measure_c5(dev, world, barrier, peak):
                          'algorithmic_bytes_per_plane': alg, 'note': 'per GPU, per plane of the chain'}}
 
 
+def dump_outputs(out, directory):
+    """Write what the last timed call returned -- the (BATCH, K, K) complex64 fields -- as float32 [..., (re, im)]:
+    focus_field_center.npy   the central 256 x 256 window of every field (8 MiB), where the PSF's energy is
+    focus_field_sample.npy   2^21 samples of the whole stack at the flat indices in
+    focus_field_index.npy    (float64, seeded, sorted; 16 MiB each)
+    so that two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    c, h = K // 2, 128
+    np.save(os.path.join(directory, 'focus_field_center.npy'),
+            torch.view_as_real(out[:, c - h:c + h, c - h:c + h]).cpu().numpy())
+    idx = np.unique(np.random.default_rng(0).integers(0, out.numel(), 1 << 21))
+    vals = out.reshape(-1)[torch.from_numpy(idx).to(out.device)]
+    np.save(os.path.join(directory, 'focus_field_sample.npy'), torch.view_as_real(vals).cpu().numpy())
+    np.save(os.path.join(directory, 'focus_field_index.npy'), idx.astype(np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # the B200 arm
 # ---------------------------------------------------------------------------------------------------------------
@@ -447,8 +466,9 @@ def run_b200(args):
     calls = max(1, args.calls_per_step)
 
     def step():  # CALLS public-API calls; each = one batched library call (pb_fft2_batch) writing 2 GiB of distinct outputs
-        for _ in range(calls):
+        for _ in range(calls - 1):
             P.focus(stack, Q)
+        return P.focus(stack, Q)
 
     def barrier():
         if world > 1:
@@ -466,11 +486,15 @@ def run_b200(args):
     barrier()
     t_start = time.perf_counter()
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         step()
+    out = step()         # only the last step's result is held, as a caller of the timed path would receive it
     e1.record()
     barrier()
     t_end = time.perf_counter()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
+    del out
     ms = e0.elapsed_time(e1)
     launches = _ops.launch_count(dev) - l0
     clocks = sampler.stop(t_start, t_end) if rank == 0 else None
@@ -600,7 +624,11 @@ def main():
     ap.add_argument('--calls-per-step', type=int, default=32,
                     help='public-API calls per step (16 propagations each); 32 makes 20 steps last >= 0.5 s')
     ap.add_argument('--no-extras', action='store_true', help='headline only (for ncu captures)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the fields the last timed call returned (rank 0; sampled, float32) to DIR/*.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -364,9 +364,45 @@ def imagechain():
     print(f'imagechain.npz written, {len(g)} arrays')
 
 
+DROPIN_KEYS = ('pupil', 'field', 'psf', 'mtf', 'free_space', 'mdft', 'czt')
+
+
+def dropin():
+    """The user code of tests/test_gpu_dropin.py (INTEGRATION.md section 1) on the reference's stock backend, fp64,
+    from the oracle's synthetic pupil (N = 512, Noll 2..11, seed 3, OPD rounded to float32): per output its max |.|,
+    the central 16 x 16 window and 2048 seeded samples, plus the reference's own fp32 error for the record."""
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__))))
+    import prysm_oracle as O
+    amp, opd32, dx = O.synthetic_pupil(512, np.float32, seed=3, nmodes=10)
+
+    def user_model():
+        opd = opd32.astype(config.precision)
+        wf = Wavefront.from_amp_and_phase(amp, opd, HeNe, dx)
+        psf = wf.focus(efl=100, Q=2)
+        inten = psf.intensity
+        out = {'pupil': wf.data, 'field': psf.data, 'psf': inten.data, 'mtf': otf.mtf_from_psf(inten).data}
+        out['free_space'] = (wf * Wavefront.phase_screen(opd * 0.1, HeNe, dx)).free_space(dz=5.0, Q=1).data
+        for kind in ('mdft', 'czt'):
+            out[kind] = wf.focus_dft(wf.prepare_executor(100.0, HeNe * 10.0 / 4, 128, kind=kind)).data
+        return out, psf.dx
+    config.precision = 32
+    r32, _ = user_model()
+    config.precision = 64
+    r64, psf_dx = user_model()
+    g = dict(psf_dx=np.float64(psf_dx), opd32_stride=opd32[::8, ::8])
+    for k in DROPIN_KEYS:
+        a = np.asarray(r64[k])
+        idx = np.sort(np.random.default_rng(len(k)).choice(a.size, 2048, replace=False))
+        g.update({f'{k}_max': np.float64(np.abs(a).max()), f'{k}_win': window(a, 16), f'{k}_idx': idx.astype(np.int32),
+                  f'{k}_val': a.ravel()[idx],
+                  f'{k}_e32': np.float64(np.abs(np.asarray(r32[k]) - a).max() / np.abs(a).max())})
+    np.savez_compressed(os.path.join(OUT, 'dropin.npz'), **g)
+    print('dropin.npz written', {k: f'{float(g[k + "_e32"]):.1e}' for k in DROPIN_KEYS})
+
+
 if __name__ == '__main__':
     os.makedirs(OUT, exist_ok=True)
-    which = sys.argv[1:] or ['small', 'full', 'full_c45', 'coronagraph', 'synthesis', 'imagechain']   # name the fixtures to (re)write
+    which = sys.argv[1:] or ['small', 'full', 'full_c45', 'coronagraph', 'synthesis', 'imagechain', 'dropin']   # name the fixtures to (re)write
     for name in which:
         {'small': small, 'full': full, 'full_c45': full_c45, 'coronagraph': coronagraph, 'synthesis': synthesis,
-         'imagechain': imagechain}[name]()
+         'imagechain': imagechain, 'dropin': dropin}[name]()

@@ -1,19 +1,19 @@
 """CPU: set_backend_to_b200() re-binds prysm's hot-path names and set_backend_to_defaults() restores them.
-Runs only where an unmodified prysm is importable (this container: /root/reference); the GPU box has no prysm."""
+Runs only where an unmodified prysm is importable: oracle/_ref (oracle/install_reference.sh) or its source tree."""
 import os
 import sys
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-_INSTALLED = os.path.join(ROOT, 'baseline', '_ref')      # baseline/install_reference.sh (the unmodified reference)
+_INSTALLED = os.path.join(ROOT, 'oracle', '_ref')
 REF = os.environ.get('PRYSM_REFERENCE', _INSTALLED if os.path.isdir(os.path.join(_INSTALLED, 'prysm')) else '/root/reference')
 
 
 @pytest.fixture()
 def prysm_pkg():
     if not os.path.isdir(os.path.join(REF, 'prysm')):
-        pytest.skip('reference prysm not present on this box')
+        pytest.skip('the reference prysm is not installed')
     sys.dont_write_bytecode = True
     sys.path.insert(0, REF)
     try:

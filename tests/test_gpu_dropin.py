@@ -3,8 +3,9 @@
 The user code below is the example of INTEGRATION.md section 1, written against `prysm` only.  It runs twice in
 the same process: once on the reference's stock numpy/scipy backend (fp64: the arbiter), once after
 `prysm_b200.mathops.set_backend_to_b200()` at precision 32 -- same objects, same calls, CUDA underneath -- and the
-results are compared at the north-star tolerance.  The reference is imported from baseline/_ref (installed by
-baseline/install_reference.sh; it travels to the GPU box with the snapshot), never from /root/reference.
+results are compared at the north-star tolerance.  The reference is imported from oracle/_ref (installed by
+oracle/install_reference.sh); where it is absent, the same user code runs on prysm_b200's own API against the
+reference's stored fp64 outputs (tests/golden/dropin.npz).
 """
 import os
 import sys
@@ -13,7 +14,7 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, 'baseline', '_ref')
+REF = os.path.join(ROOT, 'oracle', '_ref')
 
 pytestmark = pytest.mark.gpu
 
@@ -21,7 +22,7 @@ pytestmark = pytest.mark.gpu
 @pytest.fixture(scope='module')
 def prysm_ref():
     if not os.path.isdir(os.path.join(REF, 'prysm')):
-        pytest.skip('baseline/_ref is not installed (run baseline/install_reference.sh)')
+        pytest.skip('oracle/_ref is not installed (run oracle/install_reference.sh)')
     sys.path.insert(0, REF)
     try:
         import prysm
@@ -120,6 +121,66 @@ def test_user_code_on_real_prysm_matches_its_numpy_path(prysm_ref):
     w = Wavefront.from_amp_and_phase(np.ones((8, 8)), np.zeros((8, 8)), 0.5, 1.0)
     assert isinstance(w.data, np.ndarray) and isinstance(w.intensity.data, np.ndarray)
     assert not torch.is_tensor(w.focus(10, Q=2).data)
+
+
+def b200_user_model(amp, opd32):
+    """user_model's calls on prysm_b200's own classes (the same names prysm exports) at precision 32."""
+    import prysm_b200 as pb
+    from prysm_b200.propagation import Wavefront
+    from prysm_b200.otf import mtf_from_psf
+    N = amp.shape[0]
+    dx = 10.0 / N
+    wf = Wavefront.from_amp_and_phase(amp, opd32, 0.6328, dx)
+    out = {'pupil': pb.asnumpy(wf.data)}
+    psf = wf.focus(efl=100, Q=2)
+    out['field'] = pb.asnumpy(psf.data)
+    inten = psf.intensity
+    out['psf'] = pb.asnumpy(inten.data)
+    out['psf_dx'] = psf.dx
+    out['mtf'] = pb.asnumpy(mtf_from_psf(inten).data)
+    screen = Wavefront.phase_screen(opd32 * 0.1, 0.6328, dx)
+    out['free_space'] = pb.asnumpy((wf * screen).free_space(dz=5.0, Q=1).data)
+    for kind in ('mdft', 'czt'):
+        ex = wf.prepare_executor(100.0, 0.6328 * 10.0 / 4, 128, kind=kind)
+        out[kind] = pb.asnumpy(wf.focus_dft(ex).data)
+    return out
+
+
+def test_user_code_matches_reference_golden():
+    """The user code above on prysm_b200's API, against the reference's stock fp64 run stored in
+    tests/golden/dropin.npz (oracle/make_golden.py dropin): per output the central 16 x 16 window and 2048 seeded samples,
+    normalised by the stored max |.| of the full reference array."""
+    import torch
+    from conftest import load_golden
+    import prysm_oracle as O
+    import prysm_b200 as pb
+    from prysm_b200 import _ops
+    if not torch.cuda.is_available():
+        pytest.skip('needs a CUDA device')
+    g = load_golden('dropin.npz')
+    amp, opd32, _ = O.synthetic_pupil(512, np.float32, seed=3, nmodes=10)
+    assert np.array_equal(opd32[::8, ::8], g['opd32_stride'])      # the inputs the reference ran on
+    pb.config.precision = 32
+    try:
+        launches0 = _ops.launch_count()
+        got = b200_user_model(amp, opd32)
+        launches = _ops.launch_count() - launches0
+    finally:
+        pb.config.precision = 64
+    assert launches >= 10, 'the user code must run on the CUDA kernels'
+    assert abs(got['psf_dx'] - float(g['psf_dx'])) < 1e-9 * float(g['psf_dx'])
+    report = {}
+    for key, tol in (('pupil', 1e-6), ('field', 1e-6), ('psf', 1e-6), ('free_space', 1e-6), ('mdft', 1e-6), ('czt', 1e-6),
+                     ('mtf', 2e-6)):
+        a = np.asarray(got[key])
+        cy, cx = a.shape[0] // 2, a.shape[1] // 2
+        win = a[cy - 8:cy + 8, cx - 8:cx + 8]
+        diff = max(float(np.abs(win - g[f'{key}_win']).max()), float(np.abs(a.ravel()[g[f'{key}_idx']] - g[f'{key}_val']).max()))
+        # mtf: absolute (its maximum is 1); the others relative to the reference's max |.|
+        e = diff if key == 'mtf' else diff / float(g[f'{key}_max'])
+        report[key] = (e, float(g[f'{key}_e32']))
+        assert e <= tol, f'{key}: {e:.2e} from the reference fp64 result (reference fp32: {float(g[f"{key}_e32"]):.2e})'
+    print('user code vs reference fp64 golden (ours, reference fp32):', {k: (f'{a:.1e}', f'{b:.1e}') for k, (a, b) in report.items()})
 
 
 def test_elementwise_members_never_touch_numpy_exp(prysm_ref, monkeypatch):

@@ -6,14 +6,14 @@ Three runs per config on BIT-IDENTICAL inputs (built once by the reference's own
 rounded to float32 once, so that input rounding is the same on every side and the numbers below are transform error
 only):
 
-    ref64   the unmodified reference (baseline/_ref, numpy + scipy.fft), config.precision = 64   -- the arbiter
+    ref64   the unmodified reference (oracle/_ref, numpy + scipy.fft), config.precision = 64   -- the arbiter
     ref32   the same reference at config.precision = 32                                          -- its own fp32 level
     gpu32   prysm_b200 at precision 32 (complex64 kernels)
 
 Metric (SURVEY.md 8d): relative L-infinity over the FULL array, max|a - ref64| / max|ref64|, for the complex field and
 for the intensity; the RMS error over the same normaliser is given beside it because at 4096^2 = 1.7e7 samples the
-L-infinity of ANY fp32 transform chain sits ~5 sigma above its RMS.  Neither the oracle nor /root/reference is touched:
-the reference is imported from baseline/_ref (baseline/install_reference.sh).
+L-infinity of ANY fp32 transform chain sits ~5 sigma above its RMS.  The oracle is not touched:
+the reference is imported from oracle/_ref (oracle/install_reference.sh).
 """
 import argparse
 import json
@@ -25,7 +25,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, 'baseline', '_ref'))
+sys.path.insert(0, os.path.join(ROOT, 'oracle', '_ref'))
 
 HENE, EFL = 0.6328, 100.0
 
@@ -74,11 +74,11 @@ def main():
     from prysm.propagation import Wavefront as RW
     import prysm_b200 as pb
     from prysm_b200 import propagation as P
-    assert os.path.realpath(prysm.__file__).startswith(os.path.realpath(os.path.join(ROOT, 'baseline', '_ref')))
+    assert os.path.realpath(prysm.__file__).startswith(os.path.realpath(os.path.join(ROOT, 'oracle', '_ref')))
     sc = 4 if args.small else 1
     rep = {'metric': 'max|a - ref64| / max|ref64| over the full array (rel_linf) and RMS over the same normaliser',
            'inputs': 'built once by the reference in fp64, OPD / screen phase rounded to float32 once, identical on all sides',
-           'reference': f'prysm {getattr(prysm, "__version__", "0.22")} from baseline/_ref', 'configs': {}}
+           'reference': f'prysm {getattr(prysm, "__version__", "0.22")} from oracle/_ref', 'configs': {}}
     t_all = time.time()
 
     def gpu(fn):
