@@ -1,8 +1,7 @@
-// Register-resident packed-lane FFT engine shared by the tuned kernels (fft_tuned.cu, focus_fused.cu): radix-16 butterflies on
+// Register-resident packed-lane FFT engine of the tuned kernels (fft_tuned.cu): radix-16 butterflies on
 // two packed fp32 lanes, the two-exchange FFT_L skeleton, async-copy / TMA plumbing, and the geometry of the focus pipeline.
 // Everything device-side lives in an anonymous namespace (each translation unit gets its own copy).
 #pragma once
-#include <cstdlib>
 #include <algorithm>
 #include "fft_tuned.cuh"
 
@@ -148,19 +147,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                  "l"(src), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
 }
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_test(uint64_t* bar, uint32_t parity) {   // non-blocking
-    uint32_t ok;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n" : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    return ok != 0;
-}
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     asm volatile(
         "{\n"
@@ -192,9 +178,6 @@ __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, i
     asm volatile(
         "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3, %4, %5}], [%6], %7;"
         ::"r"(smem_u32(dst)), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(smem_u32(bar)), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_3d(const CUtensorMap* map, int c0, int c1, int c2) {   // into L2 only
-    asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global [%0, {%1, %2, %3}];" ::"l"(map), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void st_hint(float4* p, float4 v, uint64_t pol) {
@@ -300,7 +283,6 @@ struct FocusParams {
     long long in_bs, amp_bs, out_bs;
     // v2 pipeline
     int ntiles;             // column kernel: batch * N / T tiles, walked by a persistent grid
-    int hints;              // 1: L2 eviction hints (intermediate evict_last when written / evict_first when read, streams evict_first)
 };
 
 template <int L> struct Geo2 {
@@ -382,10 +364,10 @@ __device__ __forceinline__ void fft_two_stages_u(P2 (&v)[16], const int t, float
     sync();
 }
 
-// Row kernel, second form: ONE 512-thread CTA per SM = four independent 128-thread line groups (named barriers, own
+// Row kernel of the v2 pipeline: ONE 512-thread CTA per SM = four independent 128-thread line groups (named barriers, own
 // exchange buffer, own row buffer and mbarrier) that share the float2 twiddle plan of the column kernel in shared memory.
-// Against three 128-thread CTAs with the float4 plan in L1 (focus_row2_kernel): 16 instead of 12 warps per SM, stage-1
-// twiddles are 64-bit shared-memory loads (lane B's twiddle = lane A's times the per-thread constant w_2L^t, four scalar
+// Against an earlier form with three 128-thread CTAs per SM and the float4 plan in L1 (measured and removed, DESIGN 4.1):
+// 16 instead of 12 warps per SM, stage-1 twiddles are 64-bit shared-memory loads (lane B's twiddle = lane A's times the per-thread constant w_2L^t, four scalar
 // FP32 operations) instead of 128-bit L1 loads whose latency shows up as the kernel's top stall, and the whole unified
 // array is shared memory (no L1 working set to protect).
 template <int L> struct GeoR4 {
@@ -396,13 +378,10 @@ template <int L> struct GeoR4 {
     static constexpr size_t SMEM = BAR_OFF + 8 * sizeof(uint64_t);
 };
 
-static int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
-
 template <class K> int set_smem_attrs(Handle* h, K kernel, size_t smem, int ctas_per_sm) {
     if (!attr_needed(h, reinterpret_cast<const void*>(kernel))) return PB_OK;
     PB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int pct = (int)std::min<size_t>(100, ((size_t)ctas_per_sm * (smem + 1024) * 100 + h->max_smem_optin - 1) / h->max_smem_optin);
-    if (const char* e = getenv("PB_CARVEOUT_PCT")) pct = atoi(e);
+    const int pct = (int)std::min<size_t>(100, ((size_t)ctas_per_sm * (smem + 1024) * 100 + h->max_smem_optin - 1) / h->max_smem_optin);
     PB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
     return PB_OK;
 }

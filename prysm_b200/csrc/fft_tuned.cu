@@ -190,8 +190,9 @@ __global__ void __launch_bounds__(L / 16) focus_row_kernel(const FocusParams p) 
 //     its 4-column input tile by tensor TMA (box = 4 columns x 256 rows, 32-byte runs gathered into a contiguous
 //     [row][4] image that aliases the exchange buffers); the tile after next is requested as soon as the exchange
 //     buffers are free, so it lands while the last butterflies and the stores of the current tile run.
-//   * The row kernel gathers one intermediate row (512 runs of 32 bytes, 128 bytes apart) with two tensor-TMA boxes into
-//     the same contiguous row buffer the v1 kernel fills by a bulk copy; everything after that is the v1 code.
+//   * The row kernel (one 512-thread CTA per SM, four line groups, see GeoR4) gathers one intermediate row per group
+//     (512 runs of 32 bytes, 128 bytes apart) with two tensor-TMA boxes into a contiguous row buffer; the transform and
+//     the stores are those of the v1 row kernel.
 // =====================================================================================================
 
 
@@ -207,19 +208,14 @@ __device__ __forceinline__ void focus_col4_group(const CUtensorMap& in_map, cons
     const float2* __restrict__ plan = reinterpret_cast<const float2*>(smem4 + G4::PLAN2);
     float4* S = smem4 + (HALF * 2 + cp) * G4::XBUF;
     const SyncGroup gsync{1 + HALF, 2 * NT};
-    const uint64_t pol_tmp = l2_policy((p.hints & 1) ? 2 : 0), pol_in = l2_policy((p.hints & 1) ? 1 : 0);
+    // the intermediate is re-read by the row kernel from L2: evict_last; the input is read once: evict_first
+    const uint64_t pol_tmp = l2_policy(2), pol_in = l2_policy(1);
     auto request_tile = [&](int ww) {   // one thread: gather tile ww = (field, column tile) into the staging area
         const int fb = ww / G2::TILES, tile = ww - fb * G2::TILES;
         mbar_expect_tx(bar + 1, (uint32_t)(L * 4 * sizeof(float2)));
 #pragma unroll
         for (int b = 0; b < G2::NBOX_IN; ++b)
             tma_load_3d(smem4 + G4::STAGE + b * G2::BOXR * 2, &in_map, tile * 4, b * G2::BOXR, fb, bar + 1, pol_in);
-        const int nn = ww + gridDim.x;   // the tile after: pull it from HBM into L2 now, so that its gather is an L2 hit
-        if ((p.hints & 2) && nn < p.ntiles) {
-            const int fb2 = nn / G2::TILES, tile2 = nn - fb2 * G2::TILES;
-#pragma unroll
-            for (int b = 0; b < G2::NBOX_IN; ++b) tma_prefetch_3d(&in_map, tile2 * 4, b * G2::BOXR, fb2);
-        }
     };
     unsigned int* released = reinterpret_cast<unsigned int*>(bar + 2);   // warps that hold the inputs of the current tile, summed over tiles
     if (HALF == 0 && lt == 0) {
@@ -307,91 +303,6 @@ __global__ void __launch_bounds__(Geo4<L>::THREADS) focus_col4_kernel(const __gr
 }
 
 template <int L, bool INV>
-__global__ void __launch_bounds__(L / 16) focus_row2_kernel(const __grid_constant__ CUtensorMap tmp_map, const FocusParams p) {
-    using G = Geo<L>;
-    using G2 = Geo2<L>;
-    constexpr int NT = G::NT, R3 = G::R3, GI = G::GI;
-    constexpr uint32_t ROW_BYTES = L * sizeof(float2);
-    extern __shared__ __align__(128) unsigned char smraw[];
-    float4* S = reinterpret_cast<float4*>(smraw);                // SBUF exchange
-    float2* inb = reinterpret_cast<float2*>(S + G::SBUF);        // L-element input row
-    uint64_t* bar = reinterpret_cast<uint64_t*>(inb + L);        // 1 mbarrier
-    const int t = threadIdx.x;
-    int r = blockIdx.x;
-    const uint64_t pol_tmp = l2_policy((p.hints & 1) ? 1 : 0), pol_out = l2_policy((p.hints & 1) ? 1 : 0);
-    auto request_row = [&](int R) {   // one thread: gather intermediate row R = (field, plane, j) into `inb`
-        const int fb = R / (2 * L), rf = R - fb * (2 * L);
-        const int ph = rf / L, j = rf - ph * L;
-        const int grp = (fb * 2 + ph) * (L / 4) + (j >> 2);
-        mbar_expect_tx(bar, ROW_BYTES);
-#pragma unroll
-        for (int b = 0; b < G2::NBOX_ROW; ++b) tma_load_4d(inb + b * G2::BOXT * 4, &tmp_map, 0, j & 3, b * G2::BOXT, grp, bar, pol_tmp);
-    };
-    if (t == 0) {
-        mbar_init(bar, 1);
-        mbar_fence_init();
-        if (r < p.nrows) request_row(r);
-    }
-    __syncthreads();
-    const float sgn = ((t & 1) ? -1.0f : 1.0f) * p.scale;
-    for (int it = 0; r < p.nrows; ++it, r += gridDim.x) {
-        P2 v[16];
-        mbar_wait(bar, it & 1);
-        {
-            const float2* __restrict__ row = inb + t;
-#define PB_X(n) row[(n) * NT]
-            PB_MAKE_LANES_16(v, INV, PB_X)
-#undef PB_X
-        }
-        const int rn = r + gridDim.x;
-        auto sync_and_prefetch = [&]() {
-            __syncthreads();  // every thread holds its inputs in registers: the row buffer is free
-            if (t == 0 && rn < p.nrows) {
-                fence_proxy_async();
-                request_row(rn);
-            }
-        };
-        fft_two_stages<L, INV, 0>(v, t, S, p.plan + G::TW1, p.plan + G::TW2, sync_and_prefetch, SyncCta());
-        fft_last_stage_load<L, INV>(v, t, S);
-        __syncthreads();  // exchange buffer is free for the next row
-#pragma unroll
-        for (int g = 0; g < GI; ++g) dftR<R3, INV>(v + g * R3);
-        const int fb = r / (2 * L), rf = r - fb * (2 * L);   // field of the batch, row within its [2][L] planes
-        const int phs = rf / L, rr = rf - phs * L;
-        const int orow = (2 * rr + phs + L) & (2 * L - 1);  // fftshift along y
-        if (p.out_kind == PB_OUT_COMPLEX) {
-            float4* __restrict__ dst = reinterpret_cast<float4*>(reinterpret_cast<float2*>(p.out) + fb * p.out_bs + (long long)orow * p.out_ld);
-#pragma unroll
-            for (int g = 0; g < GI; ++g)
-#pragma unroll
-                for (int kk = 0; kk < R3; ++kk) {
-                    const int j = t + g * NT + 256 * kk;
-                    const P2 y = v[g * R3 + kk];
-                    const float4 o = INV ? make_float4(sgn * y.re.x, sgn * y.im.x, sgn * y.im.y, -sgn * y.re.y)
-                                         : make_float4(sgn * y.re.x, sgn * y.im.x, -sgn * y.im.y, sgn * y.re.y);
-                    st_hint(dst + ((j + L / 2) & (L - 1)), o, pol_out);
-                }
-        } else {
-            float2* __restrict__ dst = reinterpret_cast<float2*>(reinterpret_cast<float*>(p.out) + fb * p.out_bs + (long long)orow * p.out_ld);
-            const float2 s2 = make_float2(p.scale * p.scale, p.scale * p.scale);
-            const float2 wgt = make_float2(p.weight, p.weight);
-#pragma unroll
-            for (int g = 0; g < GI; ++g)
-#pragma unroll
-                for (int kk = 0; kk < R3; ++kk) {
-                    const int j = t + g * NT + 256 * kk;
-                    const P2 y = v[g * R3 + kk];
-                    float2 I = __fmul2_rn(s2, __ffma2_rn(y.re, y.re, __fmul2_rn(y.im, y.im)));
-                    float2* q = dst + ((j + L / 2) & (L - 1));
-                    if (p.out_kind == PB_OUT_ACCUMULATE) I = __ffma2_rn(wgt, I, ld_stream(q));
-                    st_hint(q, I, pol_out);
-                }
-        }
-    }
-}
-
-
-template <int L, bool INV>
 __global__ void __launch_bounds__(4 * L / 16) focus_row4_kernel(const __grid_constant__ CUtensorMap tmp_map, const FocusParams p) {
     using G = Geo<L>;
     using G2 = Geo2<L>;
@@ -406,7 +317,8 @@ __global__ void __launch_bounds__(4 * L / 16) focus_row4_kernel(const __grid_con
     const float2* __restrict__ plan = reinterpret_cast<const float2*>(smraw + R4::PLAN_OFF);
     uint64_t* bars = reinterpret_cast<uint64_t*>(smraw + R4::BAR_OFF);   // [0] plan, [1 + grp] row of group grp
     uint64_t* bar = bars + 1 + grp;
-    const uint64_t pol_tmp = l2_policy((p.hints & 1) ? 1 : 0), pol_out = l2_policy((p.hints & 1) ? 1 : 0);
+    // the intermediate is dead after this read, the output is not read again here: both evict_first
+    const uint64_t pol_tmp = l2_policy(1), pol_out = l2_policy(1);
     auto request_row = [&](int R) {   // one thread: gather intermediate row R = (field, plane, j) into `inb`
         const int fb = R / (2 * L), rf = R - fb * (2 * L);
         const int ph = rf / L, j = rf - ph * L;
@@ -560,8 +472,7 @@ int launch_focus(Handle* h, FocusParams p, int batch, cudaStream_t st) {
     // re-read by every line and must hit there.  (Left to itself the driver picks the 228 KB carve-out and the plan
     // streams from L2 at ~300 cycles a load.)
     const size_t unified = 256 * 1024, l1_keep = 64 * 1024;
-    int row_ctas = std::max(1, (int)((unified - l1_keep) / (smem_row + 1024)));
-    if (const char* e = getenv("PB_ROW_CTAS_PER_SM")) row_ctas = std::max(1, atoi(e));
+    const int row_ctas = std::max(1, (int)((unified - l1_keep) / (smem_row + 1024)));
     PB_TRY(set_smem_attrs(h, focus_col_kernel<L, INV, T>, smem_col, 1));
     PB_TRY(set_smem_attrs(h, focus_row_kernel<L, INV>, smem_row, row_ctas));
     PB_TRY(get_focus_plan<L>(h, &p.plan));
@@ -611,25 +522,16 @@ int launch_focus2(Handle* h, FocusParams p, int batch, cudaStream_t st) {
     using G = Geo<L>;
     using G2 = Geo2<L>;
     using G4 = Geo4<L>;
-    const size_t smem_col = G4::SMEM;
-    const size_t smem_row = (size_t)G::SBUF * sizeof(float4) + (size_t)L * sizeof(float2) + 2 * sizeof(uint64_t);
+    using R4 = GeoR4<L>;
     auto colk = focus_col4_kernel<L, INV>;
-    // resident CTAs per SM: rows -- as many as leave >= 64 KB of the unified L1/shared array as L1 (the 34 KB twiddle plan
-    // is re-read by every line and must hit there; left alone the driver picks the 228 KB carve-out and the plan streams
-    // from L2 at ~300 cycles a load); columns -- two 256-thread CTAs (the register file holds no more)
-    static const int row_ctas_env = env_int("PB_ROW_CTAS_PER_SM", 0);
-    const size_t unified = 256 * 1024, l1_keep = 64 * 1024;
-    const int row_ctas = row_ctas_env > 0 ? row_ctas_env : std::max(1, (int)((unified - l1_keep) / (smem_row + 1024)));
-    PB_TRY(set_smem_attrs(h, colk, smem_col, 1));
-    PB_TRY(set_smem_attrs(h, focus_row2_kernel<L, INV>, smem_row, row_ctas));
-    PB_TRY(get_focus_plan<L>(h, &p.plan));
-    const float4* plan_row = p.plan;
-    const float2* plan_col = nullptr;
-    PB_TRY(get_col4_plan<L>(h, &plan_col));
+    auto rowk = focus_row4_kernel<L, INV>;
+    PB_TRY(set_smem_attrs(h, colk, G4::SMEM, 1));
+    PB_TRY(set_smem_attrs(h, rowk, R4::SMEM, 1));
+    const float2* plan = nullptr;
+    PB_TRY(get_col4_plan<L>(h, &plan));
+    p.plan = reinterpret_cast<const float4*>(plan);   // both kernels read the float2 plan of Geo4
     p.nrows = batch * 2 * L;
     p.ntiles = batch * G2::TILES;
-    static const int hints = env_int("PB_FOCUS_L2_HINTS", 1);   // bit 0: eviction hints, bit 1: L2 prefetch of the tile after next
-    p.hints = hints;
     // (descriptors are copied out at once: the handle's cache may be flushed by the next lookup)
     const CUtensorMap* map = nullptr;
     CUtensorMap in_m, tmp_m;
@@ -648,17 +550,10 @@ int launch_focus2(Handle* h, FocusParams p, int batch, cudaStream_t st) {
         in_m = *map;
     }
     // column pass: one CTA per SM walks the tiles of all fields of the launch
-    p.plan = reinterpret_cast<const float4*>(plan_col);
-    colk<<<std::min(h->sm_count, p.ntiles), G4::THREADS, smem_col, st>>>(in_m, p);
+    colk<<<std::min(h->sm_count, p.ntiles), G4::THREADS, G4::SMEM, st>>>(in_m, p);
     PB_LAUNCH_CHECK(h);
-    static const int row_version = env_int("PB_ROW_V", 4);
-    if (row_version == 4) {   // four line groups per CTA, plan in shared memory
-        PB_TRY(set_smem_attrs(h, focus_row4_kernel<L, INV>, GeoR4<L>::SMEM, 1));
-        focus_row4_kernel<L, INV><<<std::min(h->sm_count, (p.nrows + 3) / 4), 4 * G::NT, GeoR4<L>::SMEM, st>>>(tmp_m, p);
-    } else {
-        p.plan = plan_row;
-        focus_row2_kernel<L, INV><<<std::min(h->sm_count * row_ctas, p.nrows), L / 16, smem_row, st>>>(tmp_m, p);
-    }
+    // row pass: one CTA per SM, four line groups per CTA, plan in shared memory
+    rowk<<<std::min(h->sm_count, (p.nrows + 3) / 4), 4 * G::NT, R4::SMEM, st>>>(tmp_m, p);
     PB_LAUNCH_CHECK(h);
     return PB_OK;
 }
@@ -691,32 +586,6 @@ __global__ void __launch_bounds__((COLS ? TP : 1) * L / 16, (RT && (!COLS || TP 
     // stall).  vin / vout: unit line stride, even pitch, 16-byte aligned base, both lines present (host: dispatch_axis_reg).
     const bool vin = COLS && (DENSE || ((p.batch_contiguous & 2) && hasB));
     const bool vout = COLS && (DENSE || ((p.batch_contiguous & 4) && hasB));
-    if (DENSE) {
-        // L2 prefetch of the lines of the CTA that will run `pf` CTAs later (= the number of resident CTAs): its input loads
-        // then hit L2 instead of paying the DRAM latency at the head of a CTA that cannot overlap loading with computing
-        const int pf = p.batch_contiguous >> 8;
-        if (pf) {
-            const int nb0 = ((int)blockIdx.x + pf) * (COLS ? TP : 1) * 2;
-            if (nb0 < p.nb) {
-                if (!COLS) {
-                    if (threadIdx.x < 2) {      // one bulk prefetch per line (contiguous: ies == 1), and of its screen row
-                        const float2* src = reinterpret_cast<const float2*>(p.in) + (long long)(nb0 + threadIdx.x) * p.ibs;
-                        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"((uint32_t)(L * sizeof(float2))) : "memory");
-                        if (PM) {
-                            const float2* sm = reinterpret_cast<const float2*>(p.pre_mat) + (long long)(nb0 + threadIdx.x) * p.pmi_bs;
-                            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(sm), "r"((uint32_t)(L * sizeof(float2))) : "memory");
-                        }
-                    }
-                } else if (c == 0) {            // the 32-byte segments (TP = 2: four columns) of the next tile, one thread per segment
-#pragma unroll
-                    for (int n = 0; n < 16; ++n) {
-                        const float2* src = reinterpret_cast<const float2*>(p.in) + (long long)nb0 * p.ibs + (long long)(n * NT + t) * p.ies;
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(src) : "memory");
-                    }
-                }
-            }
-        }
-    }
     const float2* __restrict__ in = reinterpret_cast<const float2*>(p.in);
     const float2* __restrict__ pre_e = reinterpret_cast<const float2*>(p.pre_e);
     const float2* __restrict__ pre_b = reinterpret_cast<const float2*>(p.pre_b);
@@ -969,20 +838,6 @@ int launch_axis_reg(Handle* h, const AxisPass& p, cudaStream_t st) {
     PB_TRY(get_plain_plan<L>(h, &tw1, &tw2));
     const int lines_per_cta = 2 * TP;
     const int grid = (p.nb + lines_per_cta - 1) / lines_per_cta;
-    if (DENSE) {   // L2 prefetch distance = resident CTAs (PB_AXIS_PREFETCH: bit 0 row passes, bit 1 column passes)
-        static const int pf_mode = env_int("PB_AXIS_PREFETCH", 0);
-        const size_t unified = 256 * 1024, l1_keep = 64 * 1024;
-        const int regs_ctas = COLS ? 1 : 2;
-        const int ctas = std::min<int>(regs_ctas, std::max<int>(1, (int)((unified - l1_keep) / (smem + 1024))));
-        const bool on = COLS ? (pf_mode & 2) != 0 : ((pf_mode & 1) != 0 && p.ies == 1 && (!PM || p.pmi_es == 1));
-        if (on) {
-            AxisPass q = p;
-            q.batch_contiguous = (p.batch_contiguous & 255) | ((ctas * h->sm_count) << 8);
-            axis_reg_kernel<L, INV, COLS, TP, RT, PM, DENSE><<<grid, TP * G::NT, smem, st>>>(q, tw1, tw2);
-            PB_LAUNCH_CHECK(h);
-            return PB_OK;
-        }
-    }
     axis_reg_kernel<L, INV, COLS, TP, RT, PM, DENSE><<<grid, TP * G::NT, smem, st>>>(p, tw1, tw2);
     PB_LAUNCH_CHECK(h);
     return PB_OK;
@@ -1026,8 +881,6 @@ int dispatch_axis_reg(Handle* h, const AxisPass& p0, cudaStream_t st) {
 }  // namespace
 
 int try_tuned_axis_pass(Handle* h, const AxisPass& p, cudaStream_t st) {
-    static const bool disabled = getenv("PB_DISABLE_TUNED") != nullptr || getenv("PB_DISABLE_TUNED_AXIS") != nullptr;
-    if (disabled) return PB_ERR_UNSUPPORTED;
     if (p.dtype != PB_C64 || p.in_kind == PB_IN_AMP_OPD) return PB_ERR_UNSUPPORTED;
     if (p.out_kind != PB_OUT_COMPLEX && !p.roundtrip) return PB_ERR_UNSUPPORTED;   // |.|^2 stores: round-trip epilogue only
     if (p.pre_e2 || (p.post_e2 && !p.roundtrip) || p.post_mat) return PB_ERR_UNSUPPORTED;
@@ -1042,20 +895,15 @@ int try_tuned_axis_pass(Handle* h, const AxisPass& p, cudaStream_t st) {
     }
 }
 
-// fields per launch pair: more than one evens out the tails (512 column tiles on 148 SMs = 3.46 waves; 4096 rows on
-// 444 persistent row CTAs = 9.2 rounds).  The intermediates of a group (64 MiB each at N = 2048) no longer fit L2
-// together and spill to HBM, which has the headroom: measured 87.3 / 78.8 / 76.7 / 75.7 us per field at 1 / 2 / 4 / 8.
-static int focus_fields_per_launch() {
-    static const int n = [] { const char* e = getenv("PB_FOCUS_BATCH"); return e ? std::max(1, atoi(e)) : 8; }();
-    return n;
-}
+// fields per launch pair: more than one evens out the tails (512 column tiles on 148 SMs = 3.46 waves at N = 2048).
+// The intermediates of a group (64 MiB each at N = 2048) no longer fit L2 together and spill to HBM, which has the
+// headroom: measured 87.3 / 78.8 / 76.7 / 75.7 us per field at 1 / 2 / 4 / 8.
+constexpr int FOCUS_FIELDS_PER_LAUNCH = 8;
 
 int try_tuned_fft2_batch(Handle* h, int dtype, const void* in, int in_kind, const void* amp, int amp_kind, double kturns,
                          int batch, long long in_bs, long long amp_bs, int ny, int nx, long long in_ld, int ky, int kx, int dir,
                          double scale, int shift_in, int shift_out, void* out, int out_kind, double weight, int oy, int ox,
                          long long out_ld, long long out_bs, cudaStream_t st) {
-    static const bool disabled = getenv("PB_DISABLE_TUNED") != nullptr;
-    if (disabled) return PB_ERR_UNSUPPORTED;
     if (dtype != PB_C64 || ny != nx || ky != 2 * ny || kx != 2 * nx || !shift_in || !shift_out || oy != ky || ox != kx)
         return PB_ERR_UNSUPPORTED;
     if (nx != 512 && nx != 1024 && nx != 2048) return PB_ERR_UNSUPPORTED;
@@ -1063,17 +911,10 @@ int try_tuned_fft2_batch(Handle* h, int dtype, const void* in, int in_kind, cons
     if (out_kind == PB_OUT_COMPLEX ? (out_ld & 1) || (out_bs & 1) || ((uintptr_t)out & 15) : (out_ld & 1) || (out_bs & 1) || ((uintptr_t)out & 7))
         return PB_ERR_UNSUPPORTED;  // vector stores need aligned rows
     const int N = nx;
-    // 2 = column kernel + row kernel per group of fields (default); 3 = the role-specialised single kernel of
-    // focus_fused.cu (opt-in: measured 66.4 us against 60.0 us per propagation, see DESIGN 4.1)
-    static const int version = env_int("PB_FOCUS_V", 2);
-    // v2 / v3 take their input tiles by tensor TMA: complex input, 16-byte aligned base and even pitches; everything else
-    // (the fused phase-screen input, odd pitches) runs the v1 kernels
+    // the v2 kernels take their input tiles by tensor TMA: complex input, 16-byte aligned base and even pitches (so that
+    // every group's base stays aligned); everything else (the fused phase-screen input, odd pitches) runs the v1 kernels
     const bool tma_ok = in_kind == PB_IN_COMPLEX && !((uintptr_t)in & 15) && !(in_ld & 1) && !(in_bs & 1);
-    if (version >= 3 && tma_ok) {   // stacks: one role-specialised kernel, the intermediate stays in L2 (focus_fused.cu)
-        const int rc = try_focus_fused(h, N, dir, in, in_ld, in_bs, batch, out, out_kind, out_ld, out_bs, scale, weight, st);
-        if (rc != PB_ERR_UNSUPPORTED) return rc;
-    }
-    const int per = std::min(batch, focus_fields_per_launch());
+    const int per = std::min(batch, FOCUS_FIELDS_PER_LAUNCH);
     void* tmp = nullptr;
     PB_TRY(ensure_scratch(h, 0, (size_t)per * 2 * N * N * sizeof(float2), &tmp));
     const size_t in_elt = in_kind == PB_IN_COMPLEX ? sizeof(float2) : sizeof(float);
@@ -1090,11 +931,10 @@ int try_tuned_fft2_batch(Handle* h, int dtype, const void* in, int in_kind, cons
         p.plan = nullptr;
         p.out = reinterpret_cast<char*>(out) + (size_t)b0 * out_bs * out_elt;
         p.out_ld = out_ld; p.out_kind = out_kind; p.scale = (float)scale; p.weight = (float)weight;
-        p.nrows = 0; p.ntiles = 0; p.hints = 0;
+        p.nrows = 0; p.ntiles = 0;
         p.in_bs = in_bs; p.amp_bs = amp_bs; p.out_bs = out_bs;
         int rc;
-        const bool v2_ok = tma_ok && !((uintptr_t)p.in & 15);
-        if (version >= 2 && v2_ok) {
+        if (tma_ok) {
             if (dir < 0) rc = N == 512 ? launch_focus2<512, false>(h, p, nb, st) : N == 1024 ? launch_focus2<1024, false>(h, p, nb, st) : launch_focus2<2048, false>(h, p, nb, st);
             else rc = N == 512 ? launch_focus2<512, true>(h, p, nb, st) : N == 1024 ? launch_focus2<1024, true>(h, p, nb, st) : launch_focus2<2048, true>(h, p, nb, st);
         } else if (dir < 0) rc = N == 512 ? launch_focus<512, false>(h, p, nb, st) : N == 1024 ? launch_focus<1024, false>(h, p, nb, st) : launch_focus<2048, false>(h, p, nb, st);

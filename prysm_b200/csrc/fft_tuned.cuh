@@ -18,8 +18,4 @@ int try_tuned_fft2_batch(Handle* h, int dtype, const void* in, int in_kind, cons
                          int dir, double scale, int shift_in, int shift_out, void* out, int out_kind, double weight,
                          int oy, int ox, long long out_ld, long long out_bs, cudaStream_t st);
 
-// Role-specialised single-kernel pipeline for stacks of pupils (focus_fused.cu); PB_ERR_UNSUPPORTED = not its shape
-int try_focus_fused(Handle* h, int N, int dir, const void* in, long long in_ld, long long in_bs, int batch, void* out, int out_kind,
-                    long long out_ld, long long out_bs, double scale, double weight, cudaStream_t st);
-
 }  // namespace pb

@@ -25,33 +25,28 @@
 //     output row), which brings the result under 1e-6 of the fp64 reference; the correction accumulator is
 //     2^-11 smaller and runs undrained.
 //
-// Kernel shape: one 128 x 256 output tile per CTA (UMMA M=128, N=256, K=8), 2-stage TMA -> smem ring of
-// 128-byte-swizzled K-major tiles (A_hi, A_lo 16 KB each; B_hi, B_lo 32 KB each; 96 KB per stage),
+// Kernel shape: one 128 x 256 output tile per CTA (UMMA M=128, N=256, K=8), 4-stage TMA -> smem ring of
+// 64-byte-swizzled K-major tiles (A_hi, A_lo 8 KB each; B_hi, B_lo 16 KB each; 48 KB per stage),
 // warp 0 = TMA producer, warp 1 = MMA issuer (one elected thread), warp 2 = TMEM allocator,
 // warps 4-11 = epilogue (tcgen05.ld 32x32b; lane quarter = warp % 4, column half = (warp - 4) / 4).  All 512 TMEM columns are used:
 // 256 for the main accumulator, 256 for the correction accumulator.
 #include <cuda.h>
-#include <cstdlib>
 
 #include "mdft_tc.cuh"
 
 namespace pb {
 namespace {
 
-// K extent of a pipeline stage, in fp32 = one swizzle row: 32 (128-byte swizzle, 96 KB stages, a ring of 2) or 16
-// (64-byte swizzle, 48 KB stages, a ring of 4).  The MMA of one 32-deep stage takes ~0.84 us, less than the L2 -> shared
-// latency of the next stage's 80 KB plus the lo-split behind it, and with two stages only one load is ever in flight:
-// the tensor pipe sat at 66 % (profiles/r02_ncu_mdft_summary.txt).  Four half-size stages keep three loads in flight.
-#ifndef PB_MDFT_BK
-#define PB_MDFT_BK 16
-#endif
-constexpr int BM = 128, BN = 256, BK = PB_MDFT_BK;
-static_assert(BK == 16 || BK == 32, "BK is one 64- or 128-byte swizzle row of fp32");
-constexpr int STAGES = BK == 32 ? 2 : 4;
+// K extent of a pipeline stage, in fp32 = one 64-byte swizzle row; 48 KB stages, a ring of 4.  Stages twice as deep
+// (128-byte swizzle, 96 KB, a ring of 2) were measured and dropped: the MMA of one 32-deep stage takes ~0.84 us, less than
+// the L2 -> shared latency of the next stage's 80 KB plus the lo-split behind it, and with two stages only one load is
+// ever in flight: the tensor pipe sat at 66 % (profiles/r02_ncu_mdft_summary.txt).  Four stages keep three loads in flight.
+constexpr int BM = 128, BN = 256, BK = 16;
+constexpr int STAGES = 4;
 constexpr int NTHREADS = 384;   // warp 0 TMA, 1 MMA, 2-3 TMEM alloc + TF32 lo-split converters, 4-11 epilogue
-constexpr uint32_t A_TILE = BM * BK * 4;             // 16 KB
-constexpr uint32_t B_TILE = BN * BK * 4;             // 32 KB
-constexpr uint32_t STAGE_BYTES = 2 * A_TILE + 2 * B_TILE;  // 96 KB
+constexpr uint32_t A_TILE = BM * BK * 4;             // 8 KB
+constexpr uint32_t B_TILE = BN * BK * 4;             // 16 KB
+constexpr uint32_t STAGE_BYTES = 2 * A_TILE + 2 * B_TILE;  // 48 KB
 constexpr uint32_t SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -81,14 +76,14 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
         "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar))
         : "memory");
 }
-// K-major, swizzled: rows of BK fp32 (128 or 64 B), 8-row groups 8 rows apart
+// K-major, swizzled: rows of BK fp32 (64 B), 8-row groups 8 rows apart
 __device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr) {
     uint64_t d = 0;
     d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);   // start address
     d |= (uint64_t)1 << 16;                        // leading byte offset (unused for swizzled K-major)
     d |= (uint64_t)((8 * BK * 4) >> 4) << 32;      // stride byte offset between 8-row groups
     d |= (uint64_t)1 << 46;                        // descriptor version (sm_100)
-    d |= (uint64_t)(BK == 32 ? 2 : 4) << 61;       // SWIZZLE_128B / SWIZZLE_64B
+    d |= (uint64_t)4 << 61;                        // SWIZZLE_64B
     return d;
 }
 __device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
@@ -135,10 +130,9 @@ __device__ __forceinline__ int ld_acquire_gpu(const int* p) {
 }
 
 struct GemmParams {
-    int kblocks;        // K blocks of 32 handled by one CTA
+    int kblocks;        // K blocks of BK handled by one CTA
     int chunk;          // K blocks accumulated in TMEM between drains of the main accumulator
     int mode;           // 0: write complex transposed (stage 1); 1: write fp32 transposed split-K partials
-    int conv_b;         // 1: the lo part of the B tiles is formed in shared memory too (nothing but fp32 A and B is loaded)
     float* out_hi;      // mode 0: T1^T hi as complex (float2) [N/2][ldo]; mode 1: ws [split][N][ldo]
     float* out_lo;      // mode 0: T1^T lo
     long long ldo;      // leading dimension of the transposed output, in output elements
@@ -203,11 +197,11 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_constant_
                 const uint32_t ph = (kb / STAGES) & 1;
                 mbar_wait(&empty[s], ph ^ 1);
                 unsigned char* st = smem + s * STAGE_BYTES;
-                mbar_expect_tx(&full[s], A_TILE + (p.conv_b ? B_TILE : 2 * B_TILE));
+                mbar_expect_tx(&full[s], A_TILE + 2 * B_TILE);
                 const int kc = (kb0 + kb) * BK;
                 tma_load_2d(st, &tmAhi, kc, m0, &full[s]);                 // fp32 A: read as TF32 it IS the hi part
                 tma_load_2d(st + 2 * A_TILE, &tmBhi, kc, n0, &full[s]);
-                if (!p.conv_b) tma_load_2d(st + 2 * A_TILE + B_TILE, &tmBlo, kc, n0, &full[s]);
+                tma_load_2d(st + 2 * A_TILE + B_TILE, &tmBlo, kc, n0, &full[s]);
             }
         }
     } else if (warp == 1) {
@@ -240,9 +234,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_constant_
             }
         }
     } else if (warp == 2 || warp == 3) {
-        // ===== converters: lo = x - tf32(x) for the A tile (and the B tile), element for element in the swizzled layout.
+        // ===== converters: lo = x - tf32(x) for the A tile, element for element in the swizzled layout.
         // The TF32 split used to be a streaming pre-pass over the whole input plus a second operand array; forming it on
-        // the tile in shared memory removes that pass and a third (or half) of the L2 -> SM operand traffic.
+        // the tile in shared memory removes that pass and the loads of the A_lo tiles.
         const int ct = threadIdx.x - 2 * 32;
         for (int kb = 0; kb < p.kblocks; ++kb) {
             const int s = kb % STAGES;
@@ -266,7 +260,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_constant_
                 }
             };
             split(st, st + A_TILE / 16, A_TILE / 16);
-            if (p.conv_b) split(st + 2 * A_TILE / 16, st + (2 * A_TILE + B_TILE) / 16, B_TILE / 16);
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> tensor-core (async proxy) reads
             mbar_arrive(&conv[s]);
         }
@@ -554,233 +547,6 @@ tc_gemm_sk_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_consta
     if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
 }
 
-// =====================================================================================================
-// CTA-pair form (tcgen05 cta_group::2): two CTAs of a cluster compute one 256 x 256 tile.  CTA r owns rows
-// m0 + 128 r .. of A (its own A_hi / A_lo tiles and its own 128-lane accumulators) and loads HALF of the B tile
-// (rows n0 + 128 r ..); the pair's MMA (M = 256, N = 256, issued by the leader CTA only) reads A from each CTA's own
-// shared memory and the two halves of B from both.  Per CTA and K-block the tensor core reads 96 KB of operands instead
-// of 144 KB and TMA writes 48 KB instead of 80 KB: the single-CTA kernel is bound by exactly that shared-memory
-// traffic (DESIGN 4.3).  A stage is 64 KB (96), so the ring is three deep.  Arithmetic, accumulation order and drain
-// schedule are those of tc_gemm_kernel: the results are bit-identical.
-// Synchronisation across the pair: every CTA's TMA completes on its OWN full barrier; its converter warps form A_lo
-// and then arrive (release.cluster) on the LEADER's conv barrier (4 arrivals: 2 warps x 2 CTAs); the leader's MMA
-// thread waits there, issues, and commits with multicast to BOTH CTAs' empty / tmem_full barriers; the epilogue
-// warps of both CTAs arrive on the leader's tmem_empty barrier (16 arrivals).
-// =====================================================================================================
-constexpr int STAGES2 = BK == 32 ? 3 : 6;
-constexpr uint32_t B_HALF = (BN / 2) * BK * 4;                     // 16 KB
-constexpr uint32_t STAGE2_BYTES = 2 * A_TILE + 2 * B_HALF;         // 64 KB
-constexpr uint32_t SMEM2_BYTES = STAGES2 * STAGE2_BYTES + 1024 /*align*/ + 256 /*barriers*/;
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, uint32_t rank) {   // same offset in CTA `rank` of the cluster
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {   // acquire at cluster scope
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAITC_%=:\n"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONEC_%=;\n"
-        "bra WAITC_%=;\n"
-        "DONEC_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void umma_tf32_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(d_tmem),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {   // arrives on `bar` of BOTH CTAs once the issued MMAs are done
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-                 "h"((uint16_t)3)
-                 : "memory");
-}
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
-tc_gemm_pair_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_constant__ CUtensorMap tmBhi,
-                    const __grid_constant__ CUtensorMap tmBlo, const GemmParams p) {
-    extern __shared__ unsigned char smem_raw[];
-    unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + STAGES2 * STAGE2_BYTES);
-    uint64_t* full = bars;                 // [STAGES2]  own TMA -> own converters
-    uint64_t* empty = bars + STAGES2;      // [STAGES2]  pair MMA -> own TMA producer (multicast commit)
-    uint64_t* conv = bars + 2 * STAGES2;   // [STAGES2]  converters of both CTAs -> MMA (the leader's copy is used)
-    uint64_t* tmem_full = bars + 3 * STAGES2;       // pair MMA -> own epilogue (multicast commit)
-    uint64_t* tmem_empty = bars + 3 * STAGES2 + 1;  // epilogues of both CTAs -> MMA (the leader's copy is used)
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * STAGES2 + 2);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const int m0 = blockIdx.x * BM;                 // this CTA's 128 rows (blockIdx.x = 2 * pair + rank)
-    const int n0 = blockIdx.y * BN;                 // the pair's 256 columns
-    const int nb0 = n0 + (int)rank * (BN / 2);      // the half of the B tile this CTA loads
-    const int kb0 = blockIdx.z * p.kblocks;
-    const int CHUNK = p.chunk;
-    const int nchunks = (p.kblocks + CHUNK - 1) / CHUNK;
-
-    if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tmAhi) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tmBhi) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tmBlo) : "memory");
-    }
-    if (warp == 1 && lane == 0) {
-        for (int s = 0; s < STAGES2; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); mbar_init(&conv[s], 4); }
-        mbar_init(tmem_full, 1);
-        mbar_init(tmem_empty, 16);  // one arrival per epilogue warp of the pair
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 2) {  // the same warp of both CTAs: all 512 columns in each, [0,256) main, [256,512) correction
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_slot)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    cluster_sync_all();    // barriers of both CTAs are initialised before anything arrives on them from the other side
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0) {
-        if (lane == 0) {  // ===== TMA producer (both CTAs) =====
-            for (int kb = 0; kb < p.kblocks; ++kb) {
-                const int s = kb % STAGES2;
-                const uint32_t ph = (kb / STAGES2) & 1;
-                mbar_wait_cluster(&empty[s], ph ^ 1);
-                unsigned char* st = smem + s * STAGE2_BYTES;
-                mbar_expect_tx(&full[s], A_TILE + 2 * B_HALF);
-                const int kc = (kb0 + kb) * BK;
-                tma_load_2d(st, &tmAhi, kc, m0, &full[s]);                       // fp32 A: read as TF32 it IS the hi part
-                tma_load_2d(st + 2 * A_TILE, &tmBhi, kc, nb0, &full[s]);
-                tma_load_2d(st + 2 * A_TILE + B_HALF, &tmBlo, kc, nb0, &full[s]);
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0 && rank == 0) {  // ===== MMA issuer (leader CTA only) =====
-            // instruction descriptor: D = F32, A = B = TF32, both K-major, N = 256, M = 256 (128 per CTA)
-            const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)((2 * BM) >> 4) << 24);
-            const uint32_t d_main = tmem_base, d_corr = tmem_base + 256;
-            for (int kb = 0; kb < p.kblocks; ++kb) {
-                const int s = kb % STAGES2;
-                const uint32_t ph = (kb / STAGES2) & 1;
-                const int c = kb / CHUNK, kin = kb - c * CHUNK;
-                if (kin == 0 && c > 0) {  // both epilogues must have drained the previous chunk
-                    mbar_wait_cluster(tmem_empty, (c - 1) & 1);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                }
-                mbar_wait_cluster(&conv[s], ph);   // both CTAs: TMA landed AND the converter warps wrote the lo tiles
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const uint32_t sa = smem_u32(smem + s * STAGE2_BYTES);
-                const uint64_t a_hi = make_desc(sa), a_lo = make_desc(sa + A_TILE);
-                const uint64_t b_hi = make_desc(sa + 2 * A_TILE), b_lo = make_desc(sa + 2 * A_TILE + B_HALF);
-#pragma unroll
-                for (int ks = 0; ks < BK / 8; ++ks) {
-                    const uint64_t adv = (uint64_t)(ks * 32 >> 4);  // 8 tf32 = 32 B along K inside the swizzle row
-                    umma_tf32_pair(d_main, a_hi + adv, b_hi + adv, idesc, (kin | ks) != 0);
-                    umma_tf32_pair(d_corr, a_hi + adv, b_lo + adv, idesc, (kb | ks) != 0);
-                    umma_tf32_pair(d_corr, a_lo + adv, b_hi + adv, idesc, 1u);
-                }
-                umma_commit_pair(&empty[s]);   // frees the stage in both CTAs once these MMAs have read it
-                if (kin == CHUNK - 1 || kb == p.kblocks - 1) umma_commit_pair(tmem_full);  // chunk complete, both CTAs
-            }
-        }
-    } else if (warp == 2 || warp == 3) {
-        // ===== converters (both CTAs): lo = rn_tf32(x - tf32(x)) of the own A tile, in the swizzled layout =====
-        const int ct = threadIdx.x - 2 * 32;
-        const uint32_t conv0 = mapa_u32(smem_u32(conv), 0);
-        for (int kb = 0; kb < p.kblocks; ++kb) {
-            const int s = kb % STAGES2;
-            const uint32_t ph = (kb / STAGES2) & 1;
-            mbar_wait(&full[s], ph);
-            float4* hi = reinterpret_cast<float4*>(smem + s * STAGE2_BYTES);
-            float4* lo = hi + A_TILE / 16;
-            constexpr int BATCH = 8;     // A_TILE / 16 = 1024 float4 = 2 x (64 threads x 8)
-            for (int i0 = ct; i0 < (int)(A_TILE / 16); i0 += 64 * BATCH) {
-                float4 v[BATCH];
-#pragma unroll
-                for (int j = 0; j < BATCH; ++j) v[j] = hi[i0 + 64 * j];
-#pragma unroll
-                for (int j = 0; j < BATCH; ++j)
-                    lo[i0 + 64 * j] = make_float4(tf32_rn(v[j].x - tf32_trunc(v[j].x)), tf32_rn(v[j].y - tf32_trunc(v[j].y)),
-                                                  tf32_rn(v[j].z - tf32_trunc(v[j].z)), tf32_rn(v[j].w - tf32_trunc(v[j].w)));
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> tensor-core (async proxy) reads
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(conv0 + s * 8);
-        }
-    } else if (warp >= 4) {
-        // ===== epilogue (both CTAs, each its own 128 accumulator lanes): drain chunks, then transposed stores =====
-        const int q = warp & 3;              // TMEM lane quarter this warp may access
-        const int half = (warp - 4) >> 2;    // which 128 of the 256 tile columns
-        const int m = m0 + q * 32 + lane;
-        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + half * 128;
-        const uint32_t tmem_empty0 = mapa_u32(smem_u32(tmem_empty), 0);
-        float tot[128];
-#pragma unroll
-        for (int i = 0; i < 128; ++i) tot[i] = 0.f;
-        for (int c = 0; c < nchunks; ++c) {
-            mbar_wait_cluster(tmem_full, c & 1);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-            for (int c0 = 0; c0 < 128; c0 += 16) {
-                uint32_t a[16];
-                tmem_ld16(taddr + c0, a);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-                for (int i = 0; i < 16; ++i) tot[c0 + i] += __uint_as_float(a[i]);
-            }
-            if (c + 1 < nchunks) {
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                __syncwarp();
-                if (lane == 0) mbar_arrive_cluster(tmem_empty0);
-            }
-        }
-#pragma unroll
-        for (int c0 = 0; c0 < 128; c0 += 16) {
-            uint32_t b[16];
-            tmem_ld16(taddr + 256 + c0, b);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-            for (int i = 0; i < 16; ++i) tot[c0 + i] += __uint_as_float(b[i]);
-        }
-        const int nb = n0 + half * 128;
-        if (p.mode == 0) {
-            float2* __restrict__ hi = reinterpret_cast<float2*>(p.out_hi);
-#pragma unroll
-            for (int c = 0; c < 128; c += 2) {
-                const long long o = (long long)((nb + c) >> 1) * p.ldo + m;
-                hi[o] = make_float2(tot[c], tot[c + 1]);
-            }
-        } else {
-            float* __restrict__ ws = p.out_hi + (long long)blockIdx.z * p.split_stride;
-#pragma unroll
-            for (int c = 0; c < 128; ++c) ws[(long long)(nb + c) * p.ldo + m] = tot[c];
-        }
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    cluster_sync_all();   // the leader's MMAs read the peer's shared memory: neither CTA leaves before both are done
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
-}
-
 // complex basis E (m,n) -> real expansion (2m, 2n), hi and lo
 __global__ void expand_basis_kernel(const float2* __restrict__ E, int m, int n, float* __restrict__ hi, float* __restrict__ lo) {
     const long long tot = (long long)m * n;
@@ -828,7 +594,7 @@ int make_map(Handle* h, CUtensorMap* map, const void* base, long long rows, long
     const cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)box_rows};
     const cuuint32_t estr[2] = {1, 1};
     CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), gdim, gstr, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, BK == 32 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(h, PB_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult " + std::to_string((int)r));
     return PB_OK;
@@ -875,32 +641,18 @@ int launch_gemm_sk(Handle* h, const float* A, const float* Bhi, const float* Blo
     return PB_OK;
 }
 
-// the CTA-pair form: M a multiple of 256 (pairs of 128-row tiles along x)
-int launch_gemm_pair(Handle* h, const float* A, const float* Bhi, const float* Blo, int M, int N, long long K,
-                     int splits, const GemmParams& gp, cudaStream_t st) {
-    CUtensorMap mAhi, mBhi, mBlo;
-    PB_TRY(make_map(h, &mAhi, A, M, K, BM));
-    PB_TRY(make_map(h, &mBhi, Bhi, N, K, BN / 2));
-    PB_TRY(make_map(h, &mBlo, Blo, N, K, BN / 2));
-    if (attr_needed(h, reinterpret_cast<const void*>(tc_gemm_pair_kernel)))
-        PB_CUDA(h, cudaFuncSetAttribute(tc_gemm_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM2_BYTES));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(M / BM, N / BN, splits);
-    cfg.blockDim = dim3(NTHREADS);
-    cfg.dynamicSmemBytes = SMEM2_BYTES;
-    cfg.stream = st;
-    cfg.attrs = nullptr;     // the cluster shape is compiled in (__cluster_dims__)
-    cfg.numAttrs = 0;
-    PB_CUDA(h, cudaLaunchKernelEx(&cfg, tc_gemm_pair_kernel, mAhi, mBhi, mBlo, gp));
-    PB_LAUNCH_CHECK(h);
-    return PB_OK;
+// Stream-K pays where the tile grid leaves a good part of the SMs idle and each tile is cut into 2-4 pieces (the owner's
+// gather of the other pieces stays short); it needs whole drain chunks per tile and enough chunks to spread over the SMs.
+bool use_stream_k(int tiles, int kblocks, int chunk, int sm_count) {
+    return kblocks % chunk == 0 && tiles % sm_count != 0 && 5 * tiles < 4 * sm_count && 4 * tiles >= sm_count &&
+           (long long)tiles * (kblocks / chunk) >= 4LL * sm_count;
 }
 
 int pick_splits(int ny) {
     // stage 2 has only (Mx/128)*(2My/256) tiles; split its long contraction (2*Ny) to fill the GPU
     const long long kblocks = 2LL * ny / BK;
     int s = 8;
-    while (s > 1 && (kblocks % s != 0 || kblocks / s < 4 * (32 / BK))) s >>= 1;   // at least 128 K elements per split
+    while (s > 1 && (kblocks % s != 0 || kblocks / s < 128 / BK)) s >>= 1;   // at least 128 K elements per split
     return s;
 }
 
@@ -946,57 +698,37 @@ extern "C" int pb_mdft_tc_apply(pb_handle_t hh, const void* ExB_hi, const void* 
     if (((uintptr_t)a & 15) || ((uintptr_t)work & 15)) return fail(h, PB_ERR_INVALID, "data / work must be 16-byte aligned");
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     const int splits = pick_splits(ny);
-    // 2 K-blocks (8 main accumulation steps) per drain: < 1e-6 of the fp64 result at any K (measured:
-    // 16 -> 2e-6, 8 -> 1.5e-6, 4 -> 1.2e-6, 2 -> 9e-7 on random data; the drains hide behind the L2-bound mainloop)
-    static const int chunk = [] { const char* e = getenv("PB_MDFT_CHUNK"); return (e ? std::max(1, atoi(e)) : 2) * (32 / BK); }();   // in K-blocks of BK
-    static const int conv_b = [] { const char* e = getenv("PB_MDFT_CONV_B"); return e ? atoi(e) : 0; }();
-    // PB_MDFT_PAIR=1 selects the CTA-pair kernel (cta_group::2) wherever the tile rows come in pairs.  Opt-in: bit-identical
-    // results, but the drain handshake crosses the pair and costs more than the halved operand traffic saves at the
-    // drain interval the 1e-6 budget needs (487 us against 393 us at C3 with chunk = 2; 365 us with no drains at all)
-    static const int pair = [] { const char* e = getenv("PB_MDFT_PAIR"); return e ? atoi(e) : 0; }();
+    // 64 K elements (8 main accumulation steps) per drain: < 1e-6 of the fp64 result at any K (measured, in K elements
+    // per drain: 512 -> 2e-6, 256 -> 1.5e-6, 128 -> 1.2e-6, 64 -> 9e-7 on random data; the drains hide behind the
+    // L2-bound mainloop)
+    constexpr int chunk = 2 * 32 / BK;   // in K-blocks of BK
     float* t1 = reinterpret_cast<float*>(work);
     float* ws = t1 + 2LL * ny * mx;
+    char* skw = reinterpret_cast<char*>(ws + (long long)splits * 2 * my * mx);
+    skw += (16 - ((uintptr_t)skw & 15)) & 15;
     {   // stage 1: T1^T(mx, ny) = (a @ Ex^T)^T : M = ny rows of a, N = 2*mx expanded basis rows, K = 2*nx
-        GemmParams gp{(int)(2LL * nx / BK), chunk, 0, conv_b, t1, nullptr, (long long)ny, 0};
+        GemmParams gp{(int)(2LL * nx / BK), chunk, 0, t1, nullptr, (long long)ny, 0};
         // stream-K when the tile grid leaves a good part of the SMs idle (1024^2 <-> 1024^2: 64 tiles on 148 SMs, 371 -> 346 us
         // for the coronagraph round trip); at C3 (128 tiles) it is neutral -- 358.7 against 356.5 us -- and not used.
-        // PB_MDFT_STREAMK=0 disables it, =2 forces it wherever it is legal.
-        static const int streamk = [] { const char* e = getenv("PB_MDFT_STREAMK"); return e ? atoi(e) : 1; }();
-        const int tiles1 = (ny / BM) * (2 * mx / BN);
-        const bool sk_ok = streamk && !pair && gp.kblocks % chunk == 0 && tiles1 % h->sm_count != 0 &&
-                           (streamk >= 2 || (5 * tiles1 < 4 * h->sm_count && 4 * tiles1 >= h->sm_count)) &&
-                           (long long)tiles1 * (gp.kblocks / chunk) >= 4LL * h->sm_count;
-        if (sk_ok) {
-            char* skw = reinterpret_cast<char*>(ws + (long long)splits * 2 * my * mx);
-            skw += (16 - ((uintptr_t)skw & 15)) & 15;
+        if (use_stream_k((ny / BM) * (2 * mx / BN), gp.kblocks, chunk, h->sm_count))
             PB_TRY(launch_gemm_sk(h, (const float*)a, (const float*)ExB_hi, (const float*)ExB_lo, ny, 2 * mx, 2LL * nx, gp, 1.0f, skw, st));
-        } else if (pair && ny % (2 * BM) == 0) PB_TRY(launch_gemm_pair(h, (const float*)a, (const float*)ExB_hi, (const float*)ExB_lo, ny, 2 * mx, 2LL * nx, 1, gp, st));
         else PB_TRY(launch_gemm(h, (const float*)a, (const float*)ExB_hi, (const float*)ExB_lo, ny, 2 * mx, 2LL * nx, 1, gp, st));
     }
     // stage 2: out^T' = T1^T' @ Ey'^T : M = mx, N = 2*my, K = 2*ny.  Few tiles and a long contraction: stream-K over all SMs
     // with the owner's store landing the result, scaled by `norm`, directly in (My, Mx) complex orientation (same index
     // arithmetic as stage 1's transposed complex store with ldo = mx) -- no partial planes, no reduce kernel: the 1024^2 <->
     // 1024^2 coronagraph round trip went from 340 to 249 us.  With very few tiles (C3: 16, i.e. 9 pieces per tile) the owner's
-    // serial gather costs more than it saves (373.6 against 357.6 us): those, shapes too small for it, and PB_MDFT_STREAMK=0
-    // take split-K + reduce.
+    // serial gather costs more than it saves (373.6 against 357.6 us): those, and shapes too small for it, take split-K + reduce.
     {
-        static const int streamk2 = [] { const char* e = getenv("PB_MDFT_STREAMK"); return e ? atoi(e) : 1; }();
-        static const int pair2 = [] { const char* e = getenv("PB_MDFT_PAIR"); return e ? atoi(e) : 0; }();
         const int kb2 = (int)(2LL * ny / BK);
-        const int tiles2 = (mx / BM) * (2 * my / BN);
-        if (streamk2 && !pair2 && kb2 % chunk == 0 && tiles2 % h->sm_count != 0 &&
-            (streamk2 >= 2 || (5 * tiles2 < 4 * h->sm_count && 4 * tiles2 >= h->sm_count)) &&   // 2-4 pieces per tile: the owner's gather stays short
-            (long long)tiles2 * (kb2 / chunk) >= 4LL * h->sm_count) {
-            GemmParams gp{kb2, chunk, 0, 0, reinterpret_cast<float*>(out), nullptr, (long long)mx, 0};
-            char* skw = reinterpret_cast<char*>(ws + (long long)splits * 2 * my * mx);
-            skw += (16 - ((uintptr_t)skw & 15)) & 15;
+        if (use_stream_k((mx / BM) * (2 * my / BN), kb2, chunk, h->sm_count)) {
+            GemmParams gp{kb2, chunk, 0, reinterpret_cast<float*>(out), nullptr, (long long)mx, 0};
             return launch_gemm_sk(h, t1, (const float*)EyB_hi, (const float*)EyB_lo, mx, 2 * my, 2LL * ny, gp, (float)norm, skw, st);
         }
     }
     {   // split-K partials transposed into ws[s][2my][mx]
-        GemmParams gp{(int)(2LL * ny / BK / splits), chunk, 1, conv_b, ws, nullptr, (long long)mx, 2LL * my * mx};
-        if (pair && mx % (2 * BM) == 0) PB_TRY(launch_gemm_pair(h, t1, (const float*)EyB_hi, (const float*)EyB_lo, mx, 2 * my, 2LL * ny, splits, gp, st));
-        else PB_TRY(launch_gemm(h, t1, (const float*)EyB_hi, (const float*)EyB_lo, mx, 2 * my, 2LL * ny, splits, gp, st));
+        GemmParams gp{(int)(2LL * ny / BK / splits), chunk, 1, ws, nullptr, (long long)mx, 2LL * my * mx};
+        PB_TRY(launch_gemm(h, t1, (const float*)EyB_hi, (const float*)EyB_lo, mx, 2 * my, 2LL * ny, splits, gp, st));
     }
     {
         const long long tot = (long long)my * mx;

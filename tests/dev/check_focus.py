@@ -1,4 +1,4 @@
-"""GPU: correctness of the tuned focus kernels against the oracle + timing of one variant (env-selected)."""
+"""GPU: correctness of the tuned focus kernels against the oracle + timing of the single-field and batched calls."""
 import os, sys, time
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -44,10 +44,9 @@ e0.record()
 for _ in range(reps): step()
 e1.record(); torch.cuda.synchronize()
 us = e0.elapsed_time(e1) * 1e3 / (reps * B)
-print(f'variant {os.environ.get("PB_FOCUS_PHASES_PER_LAUNCH", "1")} tuned_disabled={os.environ.get("PB_DISABLE_TUNED") is not None}: '
-      f'{us:.1f} us/propagation  {1e6 / us:.0f} prop/s  {167772160 / us / 1e3:.0f} GB/s algorithmic  frac {167772160 / us / 1e3 / 6571.2:.3f}')
+print(f'single: {us:.1f} us/propagation  {1e6 / us:.0f} prop/s  {167772160 / us / 1e3:.0f} GB/s algorithmic  frac {167772160 / us / 1e3 / 6571.2:.3f}')
 
-# batched form: all B pupils in one pb_fft2_batch call (fields share launches, PB_FOCUS_BATCH per launch pair)
+# batched form: all B pupils in one pb_fft2_batch call (fields share launches, 8 per launch pair)
 stack = torch.stack(ins)
 out_b = torch.empty((B, K, K), dtype=torch.complex64, device='cuda')
 def step_b():
@@ -60,5 +59,5 @@ e0.record()
 for _ in range(reps): step_b()
 e1.record(); torch.cuda.synchronize()
 us = e0.elapsed_time(e1) * 1e3 / (reps * B)
-print(f'batched, PB_FOCUS_BATCH={os.environ.get("PB_FOCUS_BATCH", "8 (default)")}: {us:.1f} us/propagation  {1e6 / us:.0f} prop/s  '
+print(f'batched: {us:.1f} us/propagation  {1e6 / us:.0f} prop/s  '
       f'{167772160 / us / 1e3:.0f} GB/s algorithmic  frac {167772160 / us / 1e3 / 6571.2:.3f}')

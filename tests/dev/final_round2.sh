@@ -12,5 +12,5 @@ O=gpurun_out
 ( REPS=1 timeout 500 ncu --set full --clock-control none --import-source on -k regex:axis_reg -c 12 -f -o $O/final_axis python tools/profile_axis.py > $O/final_axis_ncu.log 2>&1 )
 ( timeout 400 ncu --set full --clock-control none --import-source on -k regex:tc_gemm -s 8 -c 2 -f -o $O/final_mdft python tools/bench_mdft.py > $O/final_mdft_ncu.log 2>&1 )
 ( timeout 200 python tools/bench_paths.py > $O/final_paths.log 2>&1 )
-( timeout 200 python tools/bench_mdft.py > $O/final_mdft.log 2>&1; PB_MDFT_STREAMK=2 timeout 200 python tools/bench_mdft.py >> $O/final_mdft.log 2>&1; timeout 200 python tools/micro/tf32_peak.py >> $O/final_mdft.log 2>&1; timeout 200 python tools/bench_coronagraph.py 2>&1 | grep p32 >> $O/final_mdft.log )
+( timeout 200 python tools/bench_mdft.py > $O/final_mdft.log 2>&1; timeout 200 python tools/micro/tf32_peak.py >> $O/final_mdft.log 2>&1; timeout 200 python tools/bench_coronagraph.py 2>&1 | grep p32 >> $O/final_mdft.log )
 tail -3 $O/final_pytest.log; tail -2 $O/final_smoke.log; cat $O/final_bench_1gpu.json | cut -c1-600; tail -2 $O/final_bench_1gpu.err; cat $O/final_paths.log $O/final_mdft.log
